@@ -2,7 +2,7 @@
 """bench.py -- end-to-end frames/s of the depth -> stereo hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 1080p|4k] [--impl ours|reference]
-                    [--no-4k] [--no-cpu-baseline] [--dof S] [--exact]
+                    [--no-4k] [--no-cpu-baseline] [--dof S] [--exact] [--dump-outputs DIR]
 
 A step = one batch of `frames_per_step` synthetic frames through the hot path (DPT processor + Depth-Anything-V2
 forward + u8 depth handoff in HBM + the DIBR frame loop of render_sbs_3d + pack).  With the defaults (20 steps of
@@ -62,6 +62,8 @@ NCU_RENDER_ISSUE_ACTIVE = {"4k": 70.6, "1080p": 62.9}
 NCU_GEMM_FC1_TRAFFIC = {"vitb": 32_100_000, "vitl": None, "vits": None}
 COMMON = dict(fg=4.5, mg=-1.5, bg=-6.0, sharp=0.2, feather=10.0, ksize=9, tracking=True, floating=True,
               zps=0.01, dof=0.0)
+# --dump-outputs: elements kept per workload arm, shared between ranks (16 MB of float32; the default run has two arms)
+DUMP_ELEMS = 1 << 22
 
 
 def peaks():
@@ -360,6 +362,7 @@ class GpuArm:
 
     def step(self, mem):
         idx, wl, _lib = self._idx(), self.wl, self._lib
+        self.last_idx = idx
         if mem == _lib.MEM_DEVICE:
             a, c = self.ptr_array(self.f_dev, idx), self.ptr_array(self.o_dev, idx)
         else:
@@ -461,6 +464,19 @@ class GpuArm:
             cv2.VideoCapture, R._FrameSink = real_cap, real_sink
         return fps, n
 
+    def dump_outputs(self, out_dir):
+        """The packed output frames of the last step timed, as float32 `<workload>_frames.npy`: the flattened
+        (frames_per_step, H, W, C) stack when it fits this rank's share n of DUMP_ELEMS, else the elements at the
+        sorted unique draws of numpy default_rng(0).integers(0, size, n)."""
+        out = self.torch.stack([self.o_dev[i] for i in self.last_idx]).flatten()
+        n = DUMP_ELEMS // self.world
+        if out.numel() > n:
+            pick = np.unique(np.random.default_rng(0).integers(0, out.numel(), n))
+            out = out[self.torch.from_numpy(pick).to(self.dev)]
+        name = f"{self.key}_frames" + (f"_rank{self.rank}" if self.world > 1 else "")
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, name + ".npy"), out.float().cpu().numpy())
+
     def barrier(self):
         if self.world > 1:
             self.dist.barrier()
@@ -500,6 +516,8 @@ class GpuArm:
         ms, _ = self.timed(lambda: self.step(_lib.MEM_DEVICE), args.steps, args.warmup)
         launches = ctx.launches + deng.launches - l0 - 0
         value = world * frames / (ms / 1000.0)
+        if args.dump_outputs:  # before the arms below reuse the output buffers
+            self.dump_outputs(args.dump_outputs)
         # ---------------- end-to-end arm (pinned host buffers through the public API) ----------------
         _, e2e_s = self.timed(lambda: self.step(_lib.MEM_HOST), args.steps, args.warmup)
         clk = clocks.stop()
@@ -622,7 +640,12 @@ def main():
     ap.add_argument("--sharding", default="replicas", choices=["replicas", "exact"])
     ap.add_argument("--dof", type=float, default=None,
                     help="dof_strength (default 0 = the warp/fill/compose variant; 2.0 = the reference GUI default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output frames of the last one (a fixed sample when large) "
+                         "to DIR/<workload>_frames.npy as float32, for comparing two builds on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.sharding == "exact"):
+        ap.error("--dump-outputs covers the default GPU arm (--impl ours --sharding replicas)")
     if args.dof is not None:
         COMMON["dof"] = args.dof
     args.warmup = max(args.warmup, 3)

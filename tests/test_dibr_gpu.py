@@ -20,7 +20,7 @@ import pytest
 
 from oracle import dibr as O
 from tests.util import (BIG_NATURAL, LOOP_CASES, LOOP_CASES_EXTRA, LOOP_NATURAL, PS_CASES, PS_CASES_EXTRA, PS_NATURAL,
-                        u8_diff)
+                        load_golden, u8_diff)
 from visiondepth3d_b200.synth import synth_frame
 
 pytestmark = pytest.mark.gpu
@@ -120,7 +120,7 @@ def test_pixel_shift_vs_oracle(R, size, pi, kind, mode):
 @pytest.mark.parametrize("mode", MODES, indirect=True)
 def test_pixel_shift_vs_reference_golden(R, golden_dir, name, mode):
     c = {**PS_CASES, **PS_CASES_EXTRA}[name]
-    g = np.load(os.path.join(golden_dir, name))
+    g = load_golden(os.path.join(golden_dir, name))
     R.reset_temporal_state()
     for i in range(c["n"]):
         fr, dp = synth_frame(i, c["iw"], c["ih"], c["kind"])
@@ -136,7 +136,7 @@ def test_pixel_shift_vs_reference_golden(R, golden_dir, name, mode):
 def test_pixel_shift_natural_vs_reference(R, golden_dir, name, mode):
     """CUDA path against the UNMODIFIED reference on content off the k/255 grid: eyes <= 1 LSB, < 0.3 % flips."""
     c = PS_NATURAL[name]
-    g = np.load(os.path.join(golden_dir, name))
+    g = load_golden(os.path.join(golden_dir, name))
     R.reset_temporal_state()
     for i in range(c["n"]):
         fr, dp = synth_frame(i, c["iw"], c["ih"], c["kind"])

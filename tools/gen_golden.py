@@ -15,6 +15,7 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(__file__))
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
 import refshim  # noqa: E402
+from tests.util import save_golden  # noqa: E402
 from visiondepth3d_b200.synth import synth_frame  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(__file__), "..", "tests", "golden")
@@ -138,7 +139,7 @@ def main():
     # A. pixel_shift_cuda, identity resize, GUI-style params, 3 consecutive frames
     g = run_pixel_shift(r3d, torch, 320, 180, 320, 180, 3, "smooth",
                         blur_ksize=9, feather_strength=10.0, zero_parallax_strength=0.01)
-    np.savez_compressed(os.path.join(OUT, "ps_smooth_320x180.npz"), **g, **meta)
+    save_golden(os.path.join(OUT, "ps_smooth_320x180.npz"), **g, **meta)
     # B. 2x upsample inside pixel_shift (Half-SBS style), no floating window
     g = run_pixel_shift(r3d, torch, 320, 180, 160, 90, 2, "smooth",
                         blur_ksize=5, feather_strength=4.0, enable_floating_window=False,
@@ -289,7 +290,7 @@ def gen_natural():
                 use_floating_window=True, preserve_original_aspect=False, zero_parallax_strength=0.01)
     g = run_pixel_shift(r3d, torch, 320, 180, 320, 180, 3, "natural",
                         blur_ksize=9, feather_strength=10.0, zero_parallax_strength=0.01)
-    np.savez_compressed(os.path.join(OUT, "ps_natural_320x180.npz"), **g, **meta)
+    save_golden(os.path.join(OUT, "ps_natural_320x180.npz"), **g, **meta)
     g = run_loop(r3d, torch, cv2, 320, 180, 5, "natural", base)
     np.savez_compressed(os.path.join(OUT, "loop_natural_halfsbs_320x180.npz"), **g, **meta)
     g = run_loop(r3d, torch, cv2, 320, 180, 4, "natural", dict(base, output_format="Full-SBS", preserve_original_aspect=True))
